@@ -1,10 +1,20 @@
 #!/usr/bin/env python
 """bench.py -- Mchecks/sec of batched CheckPermission (BASELINE.json metric).
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--workload cfg3] [--impl reference]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--workload cfg3] [--impl reference] [--dump-outputs DIR]
 
 A "step" is one pass of the hot path (CheckBulkPermissions) over one batch of
 synthetic checks of the named workload (SURVEY.md 8d). Prints ONE JSON line.
+The device-resident, e2e and (N > 1) sharded legs each time exactly K steps after W (at least 3)
+warm-up steps; the sustained leg runs for --sustain-s seconds instead (0 skips it). --impl
+reference times K steps after exactly W warm-up steps.
+
+--dump-outputs DIR: after the timed steps, rank 0 writes the answers of the last timed step of every
+measured workload as DIR/<workload>_answers.npy (float32 answer codes: 1 no permission, 2 has
+permission, 255 error; one per check of the batch, at most 2^20 per workload). With --impl reference
+the file holds the oracle's answers to the first checks of the same batch, the sample it times. The
+workloads are seeded, so the same arguments give the same inputs on every run and two builds, or a
+build and the oracle, can be compared answer for answer.
 
   value     whole-job Mchecks/s, inputs resident in HBM when the timed region starts
             (zg_check_bulk_device on device buffers, CUDA events on the launch stream,
@@ -34,6 +44,9 @@ import time
 ROOT = os.path.dirname(os.path.abspath(__file__))
 if ROOT not in sys.path:
     sys.path.insert(0, ROOT)
+# bench.py writes nothing under the tree: in a writable tree, importing modules build() does not import
+# (workloads, dist) would otherwise leave their bytecode cache there
+sys.dont_write_bytecode = True
 
 _REAL_STDOUT = None
 
@@ -69,7 +82,12 @@ def parse_args():
     ap.add_argument("--sharded-timeout", type=float, default=300.0, help="hard limit of the sharded leg, seconds")
     ap.add_argument("--sustain-s", type=float, default=2.5,
                     help="length of the back-to-back 'sustained' leg of the primary workload (0 = skip)")
-    return ap.parse_args()
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="write the answers of the last timed step of each workload as DIR/<workload>_answers.npy")
+    args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    return args
 
 
 def host_cores():
@@ -195,8 +213,11 @@ def cpu_reference_arm(args, rank, world):
         o.check_bulk(sample, nthreads=cores)
     t0 = time.perf_counter()
     for _ in range(args.steps):
-        o.check_bulk(sample, nthreads=cores)
+        answers = o.check_bulk(sample, nthreads=cores)
     dt = time.perf_counter() - t0
+    if args.dump_outputs:
+        os.makedirs(args.dump_outputs, exist_ok=True)
+        np.save(os.path.join(args.dump_outputs, f"{w.name}_answers.npy"), answers.astype(np.float32))
     val = n * args.steps / dt / 1e6
     desc = f"first {n} checks of the {w.name} batch per step, {cores} threads"
     emit({
@@ -277,6 +298,7 @@ def measure_workload(name, args, rank, local_rank, world, dist, primary, sampler
         dist.barrier()
     dev_ms = sum(a.elapsed_time(b) for a, b in evs)
     launches = eng.stats()["launches"] - launches0
+    last_answers = d_out.cpu().numpy() if (args.dump_outputs and rank == 0) else None
     t = torch.tensor([dev_ms], dtype=torch.float64, device="cuda")
     if dist:
         dist.all_reduce(t, op=dist.ReduceOp.MAX)
@@ -318,21 +340,20 @@ def measure_workload(name, args, rank, local_rank, world, dist, primary, sampler
     pin_in = zgpu._lib.PinnedArray(n, zgpu.CHECK_DTYPE)
     pin_out = zgpu._lib.PinnedArray(n, np.uint8)
     pin_in.array[:] = items
-    for _ in range(2):
+    for _ in range(warmup):
         eng.check_bulk_ptr(pin_in.ptr, n, pin_out.ptr)
-    e2e_steps = max(3, min(steps, 50))
     if dist:
         dist.barrier()
     torch.cuda.synchronize()
     t0 = time.perf_counter()
-    for _ in range(e2e_steps):
+    for _ in range(steps):
         eng.check_bulk_ptr(pin_in.ptr, n, pin_out.ptr)
     torch.cuda.synchronize()
     e2e_s = time.perf_counter() - t0
     t = torch.tensor([e2e_s], dtype=torch.float64, device="cuda")
     if dist:
         dist.all_reduce(t, op=dist.ReduceOp.MAX)
-    e2e_value = n * world * e2e_steps / float(t.item()) / 1e6
+    e2e_value = n * world * steps / float(t.item()) / 1e6
     clocks = sampler.stop() if (sampler is not None and rank == 0) else None
     host_answers = pin_out.array.copy()
     assert np.array_equal(host_answers, d_out.cpu().numpy()), "host and device entry points disagree"
@@ -383,7 +404,7 @@ def measure_workload(name, args, rank, local_rank, world, dist, primary, sampler
             "value": value, "unit": UNIT, "ms_per_step": kernel_ms,
             "config": workload_config(w, args, world),
             "e2e": {"value": e2e_value, "unit": UNIT, "h2d_bytes_per_step": n * 16, "d2h_bytes_per_step": n,
-                    "steps": e2e_steps, "api": "zg_check_bulk (C ABI, pinned host buffers)"},
+                    "steps": steps, "api": "zg_check_bulk (C ABI, pinned host buffers)"},
             "gpu_launches": int(launches),
             "roofline": {"bound": bound_from_evidence(dram_frac, achieved / peak), "achieved": achieved, "peak": peak,
                          "unit": "GB/s", "frac": achieved / peak, "traffic": traffic, "dram_gbs": dram_gbs,
@@ -406,6 +427,9 @@ def measure_workload(name, args, rank, local_rank, world, dist, primary, sampler
             out["sustained"] = sustained
         if clocks is not None:
             out["clocks"] = clocks
+    if last_answers is not None:
+        os.makedirs(args.dump_outputs, exist_ok=True)
+        np.save(os.path.join(args.dump_outputs, f"{w.name}_answers.npy"), last_answers.astype(np.float32))
     del d_items, d_out, flush, pin_in, pin_out
     eng.close()
     torch.cuda.empty_cache()
@@ -437,7 +461,8 @@ def measure_sharded(args, rank, local_rank, world, dist):
     d_items = torch.from_numpy(mine.view(np.uint8).copy()).cuda()
     ck = zdist.DeviceShardedChecker(eng, zdist.TorchDeviceTransport())
     chunk = 1 << 18  # checks per rank per round: bounds the sub-queries a pass may raise (~20 per check, buffer 16 M)
-    steps = max(2, min(args.steps, 5))
+    n_chunks = (hi - lo + chunk - 1) // chunk
+    steps, warmup = args.steps, max(args.warmup, 3)
 
     def one_step():
         outs = []
@@ -447,8 +472,10 @@ def measure_sharded(args, rank, local_rank, world, dist):
         return torch.cat(outs)
 
     note(f"shard published: {eng.stats()['tuples']} relationships")
-    ans = one_step()  # warm-up
-    note(f"first step done: levels {ck.stats['levels']}, sub-queries sent {ck.stats['subqueries_sent']}")
+    for i in range(warmup):
+        ans = one_step()
+        if i == 0:
+            note(f"first step done: levels {ck.stats['levels']}, sub-queries sent {ck.stats['subqueries_sent']}")
     dist.barrier()
     torch.cuda.synchronize()
     t0 = time.perf_counter()
@@ -482,12 +509,12 @@ def measure_sharded(args, rank, local_rank, world, dist):
         want = rep.check_bulk(items)
         mism = int((full != want).sum())
         rep.close()
-        rounds = steps * ((hi - lo + chunk - 1) // chunk)
+        passes = warmup + steps  # the checker's counters include the warm-up steps
         out = {"value": items.size * steps / dt / 1e6, "unit": UNIT, "ms_per_step": dt / steps * 1e3, "steps": steps,
-               "mismatches_vs_replica": mism, "tuples_over_all_shards": int(n_tuples_owned.item()),
-               "levels": st["levels"], "subqueries_per_check": st["subqueries_sent"] / max((hi - lo) * (steps + 1), 1),
-               "exchanges_per_round": st["exchanges"] / max(rounds + (hi - lo + chunk - 1) // chunk, 1),
-               "bytes_sent_per_rank_per_step": st["bytes_sent"] / (steps + 1),
+               "warmup": warmup, "mismatches_vs_replica": mism, "tuples_over_all_shards": int(n_tuples_owned.item()),
+               "levels": st["levels"], "subqueries_per_check": st["subqueries_sent"] / max((hi - lo) * passes, 1),
+               "exchanges_per_round": st["exchanges"] / max(passes * n_chunks, 1),
+               "bytes_sent_per_rank_per_step": st["bytes_sent"] / passes,
                "limiting": "per-level round trip (kernel pass + count exchange + NCCL all-to-all): latency-bound, "
                            "bytes are far below NVLink",
                "config": {"workload": f"cfg4 object-hash sharded x{world}: {w.note}", "chunk_checks_per_rank": chunk,
@@ -513,26 +540,30 @@ def run_sharded_leg(args, rank, world, dist):
     # under torchrun the workers use the AGENT's store; the children form their own group: rank 0's child hosts it
     env["TORCHELASTIC_USE_AGENT_STORE"] = "False"
     env["ZGPU_SHARDED_OUT"] = out_path
-    log_dir = os.path.join(ROOT, "gpurun_out")
-    os.makedirs(log_dir, exist_ok=True)
     cmd = [sys.executable, os.path.abspath(__file__), "--sharded-child", "--gpus", str(world), "--steps", str(args.steps),
            "--warmup", str(args.warmup)]
     err = None
-    log_path = os.path.join(log_dir, f"sharded_child_rank{rank}.log")
-    try:
-        with open(log_path, "w") as lf:
+    with tempfile.TemporaryFile() as lf:  # the child's log: relayed to this rank's stderr, its tail into the error
+        try:
             r = subprocess.run(cmd, env=env, timeout=args.sharded_timeout, stdout=lf, stderr=subprocess.STDOUT)
-        if r.returncode != 0:
-            with open(log_path) as lf:
-                err = f"child rc={r.returncode}: {lf.read()[-300:]}"
-    except subprocess.TimeoutExpired:
-        err = f"child timed out after {args.sharded_timeout} s (see {log_path})"
+            if r.returncode != 0:
+                err = f"child rc={r.returncode}"
+        except subprocess.TimeoutExpired:
+            err = f"child timed out after {args.sharded_timeout} s (raise --sharded-timeout or lower --steps)"
+        lf.seek(0)
+        log = lf.read().decode(errors="replace")
+    sys.stderr.write(log)
+    sys.stderr.flush()
+    if err:
+        err += ": " + log[-300:]
     dist.barrier()
     if rank != 0:
         return None
     if os.path.exists(out_path):
         with open(out_path) as f:
-            return json.load(f)
+            res = json.load(f)
+        os.remove(out_path)
+        return res
     return {"error": err or "no result"}
 
 

@@ -7,7 +7,6 @@ timeout 900 python -m torch.distributed.run --nnodes=1 --nproc-per-node $n --mas
 echo "bench rc=$?"; tail -3 gpurun_out/${tag}_bench_n${n}.err | cut -c1-300
 python -c "
 import json; b=json.load(open('gpurun_out/${tag}_bench_n${n}.json')); print('value', b['value'], 'e2e', b['e2e']['value']); print(json.dumps(b.get('configs',{}).get('cfg4_sharded'))[:1200])"
-tail -12 gpurun_out/sharded_child_rank0.log 2>/dev/null | cut -c1-300
 for sc in $scale; do
   timeout 900 python scripts/cfg5_replay.py --devices $n --clients 1000 --scale $sc --rounds 2 > gpurun_out/${tag}_cfg5_n${n}_s${sc}.json 2> gpurun_out/${tag}_cfg5_n${n}_s${sc}.err
   echo "cfg5 scale $sc rc=$?"; tail -3 gpurun_out/${tag}_cfg5_n${n}_s${sc}.err | cut -c1-300; cut -c1-1400 gpurun_out/${tag}_cfg5_n${n}_s${sc}.json
